@@ -9,8 +9,9 @@ One "step" = one training iteration's worth of the hot path on one batch of synt
 value = shadow rays processed per second over the whole job (fwd + bwd rays, all ranks), in Mrays/s;
 a ray is counted the way the reference traces it: covered pixels x 2 N^2 per pass (SURVEY.md section 8d).
 
-Usage (driver contract):  python bench.py --gpus N --steps K --warmup W          (torchrun for N > 1)
-                          python bench.py --impl reference ...                    (CPU oracle arm)
+Usage:  python bench.py --gpus N --steps K --warmup W          (torchrun for N > 1)
+        python bench.py --impl reference ...                    (CPU oracle arm)
+        python bench.py ... --dump-outputs DIR                  (also save the last timed step's outputs as DIR/<name>.npy)
 """
 import argparse
 import json
@@ -19,6 +20,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True         # the benchmark may run from a read-only tree: no __pycache__ next to the sources
 
 import numpy as np
 
@@ -297,8 +300,21 @@ class GpuWorkload:
     def run(self):
         if self.graph is not None:
             self.graph.replay()
-            return self.graph_loss
-        return self.step()
+            self.loss = self.graph_loss
+        else:
+            self.loss = self.step()
+        return self.loss
+
+    def dump_outputs(self, out_dir):
+        """Save what the last run() handed its caller -- the loss, the updated trainable parameters (light probe, kd / ks textures)
+        and their gradients -- as float32 `out_dir/<name>.npy` (~52 MB for the default workload)."""
+        os.makedirs(out_dir, exist_ok=True)
+        arrays = {"loss": self.loss.detach().reshape(1)}
+        for i, (name, p) in enumerate(zip(("light", "kd_tex", "ks_tex"), self.bucket.params)):
+            arrays[name] = p.detach()
+            arrays[name + "_grad"] = self.flat_grad[self.bucket.offsets[i]:self.bucket.offsets[i + 1]].view(p.shape)
+        for name, t in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def time_env_kernels(w, reps=20, warm=5, full=False, shadow_scale=1.0):
@@ -607,13 +623,15 @@ def quiet_stdout():
     os.dup2(2, 1)
 
 
-def hard_exit():
-    """Leave without tearing down NCCL communicators / captured graphs: with the all-reduce captured inside CUDA graphs,
+def finish(world):
+    """End the run.  One process: return, so the interpreter shuts down normally (exit handlers run, libraries are unloaded).
+    Several ranks: leave without tearing down NCCL communicators / captured graphs -- with the all-reduce captured inside CUDA graphs,
     `destroy_process_group()` was observed to block for minutes after the result line had been printed (rank 0 works alone on the
     parity / CPU legs long after the other ranks are done).  All results are flushed; the OS reclaims the rest."""
     sys.stdout.flush()
     sys.stderr.flush()
-    os._exit(0)
+    if world > 1:
+        os._exit(0)
 
 
 def emit(obj):
@@ -622,6 +640,8 @@ def emit(obj):
         os.dup2(_STDOUT_FD, 1)
     print(json.dumps(obj))
     sys.stdout.flush()
+    if _STDOUT_FD is not None:
+        os.dup2(2, 1)                  # whatever is printed while the process shuts down stays off the result line's stream
 
 
 def timed_loop(w, steps, barrier, torch):
@@ -703,7 +723,13 @@ def main():
     ap.add_argument("--mesh", default=None, help="override mesh: blob | blob+torus | full | bob-like | grid1m (debug)")
     ap.add_argument("--level", type=int, default=None, help="override icosphere subdivision level (debug)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save the loss, parameters and gradients of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the outputs of the GPU step; the reference arm has none to save")
     quiet_stdout()
     wl = dict(WORKLOAD)
     if args.views:
@@ -796,6 +822,8 @@ def main():
     ms = timed_loop(w, args.steps, barrier, torch)
     clk.end()
     clk.close()
+    if args.dump_outputs and rank == 0:
+        w.dump_outputs(args.dump_outputs)
     ms_step = max_over_ranks(ms, world, dev, torch, dist) / args.steps
     rays_pass_all = sum_over_ranks(w.rays_per_pass, world, dev, torch, dist)
     rays_min = -max_over_ranks(-float(w.rays_per_pass), world, dev, torch, dist)
@@ -899,7 +927,7 @@ def main():
         barrier()
 
     if rank != 0:
-        hard_exit()
+        return finish(world)
 
     # ---- rank 0: parity of this launch configuration, roofline of the dominant kernel, CPU baseline -----------------------------
     parity = None
@@ -997,7 +1025,7 @@ def main():
         "cpu_baseline": cpu,
     }
     emit(out)
-    hard_exit()
+    finish(world)
 
 
 if __name__ == "__main__":

@@ -13,9 +13,12 @@ Two builds of the same source exist: fp32 (the oracle proper, ``Oracle()``) and 
 (``Oracle(f64=True)``), the latter used only to validate the hand-derived adjoints by finite
 differences.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -40,12 +43,17 @@ def _cpu_has_fma():
 
 
 def build(force=False):
-    """Compile the C restatement with gcc (fp32 + fp64 variants). -ffp-contract=off is mandatory."""
+    """Compile the C restatement with gcc (fp32 + fp64 variants). -ffp-contract=off is mandatory.  In a read-only tree (a
+    benchmark run from an installed checkout) a library that has to be (re)built goes to a fresh temporary directory instead."""
+    global _BUILD
+    fresh = lambda p: os.path.exists(p) and all(os.path.getmtime(p) >= os.path.getmtime(s) for s in _SRC)
+    todo = [f64 for f64 in (False, True) if force or not fresh(_lib_path(f64))]
+    if todo and not os.access(_BUILD if os.path.isdir(_BUILD) else _HERE, os.W_OK):
+        _BUILD, todo = tempfile.mkdtemp(prefix="mcoracle-"), [False, True]
+        atexit.register(shutil.rmtree, _BUILD, True)        # a loaded library stays mapped after its file is removed
     os.makedirs(_BUILD, exist_ok=True)
-    for f64 in (False, True):
+    for f64 in todo:
         out = _lib_path(f64)
-        if not force and os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(s) for s in _SRC):
-            continue
         cmd = ["gcc", "-O2", "-ffp-contract=off", "-fopenmp", "-shared", "-fPIC", "-o", out, _SRC[0], "-lm"]
         if _cpu_has_fma():
             cmd.insert(2, "-mfma")       # only the explicit fmaf()/fma() calls of mt_eval use it (contraction stays off)

@@ -26,6 +26,30 @@ def rel_l2(a, b):
     return float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-30))
 
 
+def pick(a, k=128, keep=()):
+    """A fixed sample of the rows (pixels, texels, rays) of `a` over all but its last dimension: at most k evenly spaced rows plus
+    every row listed in `keep` (flat row indices of the inputs a test plants on purpose).  Only the frozen reference outputs too large
+    to store whole are stored at these rows; all of `a` when it has no more than k rows."""
+    a = np.asarray(a)
+    rows = a.reshape(-1, a.shape[-1])
+    even = np.linspace(0, rows.shape[0] - 1, min(k, rows.shape[0])).round().astype(np.int64)
+    return rows[np.unique(np.concatenate([even, np.asarray(keep, np.int64)]))]
+
+
+FROZEN_REFERENCE = os.path.join(ROOT, "tests", "golden", "ref_compiled_kernels.npz")
+_FROZEN = {}
+
+
+def frozen_reference(case):
+    """The frozen outputs of the reference's own kernels for one test case (tests/golden/make_ref_kernels_golden.py): {field: array}."""
+    if not _FROZEN:
+        with np.load(FROZEN_REFERENCE) as z:
+            for key in z.files:
+                c, field = key.split("|", 1)
+                _FROZEN.setdefault(c, {})[field] = z[key]
+    return _FROZEN[case]
+
+
 def make_case(res=32, B=1, N=4, mesh="blob+torus", level=2, light="random", light_hw=(32, 64), seed=0, ks_mode="random",
               perm_rows=512, closest=None):
     """Returns a dict of numpy arrays describing one env_shade problem.

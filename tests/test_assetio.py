@@ -63,14 +63,20 @@ def test_obj_roundtrip_and_polygons(tmp_path):
     assert m["t_tex_idx"].tolist() == [[0, 1, 2], [0, 2, 3], [0, 1, 2]] and np.allclose(m["v_tex"][3], [0, 0.75])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data/irrmaps/aerodynamics_workshop_2k.hdr"), reason="reference assets only exist in the build container")
 def test_reads_the_reference_assets_when_present():
-    img = assetio.load_hdr("/root/reference/data/irrmaps/aerodynamics_workshop_2k.hdr")
-    assert img.shape == (1024, 2048, 3) and np.isfinite(img).all() and img.min() >= 0 and img.max() > 10
-    m = assetio.load_obj("/root/reference/data/spot/spot.obj")
-    assert m["t_pos_idx"].shape == (5856, 3) and m["v_pos"].shape[0] == 2930       # SURVEY section 2: spot = 2 930 verts / 5 856 tris
-    b = assetio.load_obj("/root/reference/data/bob/bob_tri.obj")
-    assert b["t_pos_idx"].shape == (10688, 3)
+    """Real files of the reference's data set, cut down to fixtures by tests/golden/make_asset_fixtures.py: the probe header with two of
+    its run-length encoded scanlines (aerodynamics_workshop_2k.hdr, rows 0-1) and the first 64 faces of spot.obj with the lines they use."""
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    img = assetio.load_hdr(os.path.join(golden, "probe_rows2.hdr"))
+    assert img.shape == (2, 2048, 3) and img.dtype == np.float32 and np.isfinite(img).all() and img.min() >= 0
+    # rows 0-1 of the full 1024 x 2048 probe decode to these values (sum in float64, max)
+    assert abs(img.astype(np.float64).sum() / 588.616943359375 - 1) < 1e-9 and img.max() == np.float32(0.07666015625)
+    m = assetio.load_obj(os.path.join(golden, "spot_head.obj"))
+    assert m["v_pos"].shape == (74, 3) and m["v_tex"].shape == (74, 2) and m["v_nrm"].shape == (74, 3)
+    for k in ("t_pos_idx", "t_tex_idx", "t_nrm_idx"):
+        assert m[k].shape == (64, 3) and m[k].min() == 0 and m[k].max() == 73, k
+    assert m["mtllib"] == "spot.mtl" and m["usemtl"] == [("initialShadingGroup", 0)]
+    assert np.abs(np.linalg.norm(m["v_nrm"], axis=-1) - 1).max() < 1e-3 and (m["v_tex"] >= 0).all() and (m["v_tex"] <= 1).all()
 
 
 def test_mtl_roundtrip_and_reference_asset(tmp_path):
@@ -85,10 +91,9 @@ def test_mtl_roundtrip_and_reference_asset(tmp_path):
     (tmp_path / "c.mtl").write_text("# comment\nnewmtl a\nKd 0.1 0.2 0.3 # trailing\nbump -bm 1.0 n.png\nillum 2\n")
     c = assetio.load_mtl(str(tmp_path / "c.mtl"))[0]
     assert np.allclose(c["kd"], [0.1, 0.2, 0.3]) and c["bump"] == "n.png" and c["illum"][0] == 2
-    ref = "/root/reference/data/spot/metal.mtl"
-    if os.path.exists(ref):                               # build container only; the GPU box has no /root/reference
-        m = assetio.load_mtl(ref)
-        assert len(m) >= 1 and "ks" in m[0] or "map_ks" in m[0]
+    m = assetio.load_mtl(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "spot_metal.mtl"))   # the reference's data/spot/metal.mtl
+    assert len(m) == 1 and m[0]["name"] == "initialShadingGroup" and m[0]["bsdf"] == "pbr" and m[0]["map_kd"] == "spot_texture.png"
+    assert np.array_equal(m[0]["ks"], np.float32([0.0, 0.2, 1.0]))
 
 
 @pytest.mark.parametrize("shape,dtype", [((17, 23), np.uint8), ((9, 31, 3), np.uint8), ((8, 8, 4), np.uint8), ((5, 7, 2), np.uint8), ((6, 10, 3), np.uint16), ((4, 4), np.uint16)])

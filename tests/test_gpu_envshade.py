@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from common import make_case, oracle, rel_l2
+from common import make_case, oracle, pick, rel_l2
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -264,41 +264,56 @@ def test_tiny_and_flat_meshes(dev, n_occ):
     assert rel_l2(diff.cpu().numpy(), d_ref) < TOL and rel_l2(spec.cpu().numpy(), s_ref) < TOL
 
 
+def _compiled_reference_case():
+    c = make_case(res=24, B=2, N=4, seed=3)
+    ra = (c["scene"], c["mask"], c["ro"], c["pos"], c["nrm"], c["view"], c["kd"], c["ks"], c["light"], c["pdf"], c["rows"], c["cols"], c["perms"])
+    g = np.random.default_rng(1)
+    gd = g.uniform(size=c["pos"].shape).astype(np.float32); gs = g.uniform(size=c["pos"].shape).astype(np.float32)
+    return c, ra, gd, gs
+
+
+GRAD_NAMES = ("pos", "nrm", "kd", "ks", "light")
+
+
+def ref_product_case(ref, bsdf):
+    """What the reference's raygen program returns for test_product_against_the_compiled_reference (frozen in tests/golden)."""
+    c, ra, gd, gs = _compiled_reference_case()
+    d_r, s_r = ref.env_shade(*ra, BSDF=bsdf, n_samples_x=4, rnd_seed=9)
+    g_r = ref.env_shade(*ra, BSDF=bsdf, n_samples_x=4, rnd_seed=9, grads=(gd, gs))
+    out = dict(diff=pick(d_r), spec=pick(s_r), **{n: pick(g) for n, g in zip(GRAD_NAMES, g_r)})
+    out.update({n + "_absmax": np.abs(g).max() for n, g in zip(GRAD_NAMES, g_r)})
+    return out
+
+
 @pytest.mark.parametrize("bsdf", ["pbr", "diffuse"])
 def test_product_against_the_compiled_reference(dev, bsdf):
-    """The CUDA path against the REFERENCE's own raygen program (oracle/_ref: kernel.cu compiled unmodified for the host, prebuilt in the
-    build container, shadow rays answered by the oracle's predicate).  Radiance within 1e-4; gradients within the fp32 noise floor that
-    separates the reference itself from the fp64 evaluation of the same samples."""
+    """The CUDA path against the REFERENCE's own raygen program (kernel.cu compiled unmodified for the host, shadow rays answered by the
+    oracle's predicate), whose outputs are frozen in tests/golden/ref_compiled_kernels.npz at a fixed sample of pixels / texels.
+    Radiance within 1e-4; gradients within the fp32 noise floor that separates the reference itself from the fp64 evaluation of the
+    same samples."""
     import nvdiffrecmc_b200.optixutils as ou
-    from oracle import Reference
-    try:
-        ref = Reference(oracle())
-    except RuntimeError as e:
-        pytest.skip(str(e))
+    from common import frozen_reference
     N = 4
-    c = make_case(res=24, B=2, N=N, seed=3)
+    c, ra, gd, gs = _compiled_reference_case()
+    r_ref = frozen_reference("product-" + bsdf)
     ctx = _ctx(c, dev)
     a = _args(c, dev)
     for i in (2, 3, 5, 6, 7):
         a[i].requires_grad_(True)                                       # pos, nrm, kd, ks, light
     diff, spec = ou.optix_env_shade(ctx, *a, BSDF=bsdf, n_samples_x=N, rnd_seed=9, perms=_t(c, "perms", dev))
-    ra = (c["scene"], c["mask"], c["ro"], c["pos"], c["nrm"], c["view"], c["kd"], c["ks"], c["light"], c["pdf"], c["rows"], c["cols"], c["perms"])
-    d_r, s_r = ref.env_shade(*ra, BSDF=bsdf, n_samples_x=N, rnd_seed=9)
-    assert rel_l2(diff.detach().cpu().numpy(), d_r) < TOL
+    assert rel_l2(pick(diff.detach().cpu().numpy()), r_ref["diff"]) < TOL
     if bsdf == "pbr":
-        assert rel_l2(spec.detach().cpu().numpy(), s_r) < TOL
-    g = np.random.default_rng(1)
-    gd = g.uniform(size=d_r.shape).astype(np.float32); gs = g.uniform(size=d_r.shape).astype(np.float32)
+        assert rel_l2(pick(spec.detach().cpu().numpy()), r_ref["spec"]) < TOL
     torch.autograd.backward([diff, spec], [torch.tensor(gd, device=dev), torch.tensor(gs, device=dev)])
-    g_r = ref.env_shade(*ra, BSDF=bsdf, n_samples_x=N, rnd_seed=9, grads=(gd, gs))
     o64 = oracle(f64=True)
     g64 = o64.env_shade(o64.scene(c["verts"], c["tris"]), *ra[1:], BSDF=bsdf, n_samples_x=N, rnd_seed=9, grads=(gd, gs),
                         sampling_gbuffer=(c["pos"], c["nrm"], c["kd"], c["ks"]))
-    for name, t, r, r64 in zip(("pos", "nrm", "kd", "ks", "light"), (a[2], a[3], a[5], a[6], a[7]), g_r, g64):
-        got = t.grad.cpu().numpy() if t.grad is not None else np.zeros_like(r)
-        if np.abs(r).max() == 0:
+    for name, t, r64 in zip(GRAD_NAMES, (a[2], a[3], a[5], a[6], a[7]), g64):
+        got = t.grad.cpu().numpy() if t.grad is not None else np.zeros_like(r64)
+        if r_ref[name + "_absmax"] == 0:
             assert np.abs(got).max() == 0, name
             continue
+        got, r, r64 = pick(got), r_ref[name], pick(r64)
         floor = rel_l2(r, r64)                                          # how far the fp32 reference is from exact arithmetic here
         assert rel_l2(got, r) < max(TOL, 2.0 * floor), (name, rel_l2(got, r), floor)
 
