@@ -19,7 +19,6 @@
 //     share one pass (NSIG = 2): weights are computed once.
 #include "common.cuh"
 #include <cuda.h>          // CUtensorMap + the cuTensorMapEncodeTiled prototype (resolved at run time through cudaGetDriverEntryPoint: no libcuda link)
-#include <stdlib.h>
 
 namespace {
 
@@ -327,8 +326,7 @@ static int launch_bilateral_tma(const mcs_tensor *nrm, const mcs_tensor *zdz, co
                                 cudaStream_t stream)
 {
     constexpr int CS = BWD ? 4 : 3;
-    static const bool disabled = getenv("MCS_DENOISE_NO_TMA") != nullptr;       // developer switch: same-library A/B, tests of the plain path
-    if (disabled || tma_encoder() == nullptr) return 1;
+    if (tma_encoder() == nullptr) return 1;
     if (!(tma_ok(nrm, 3) && tma_ok(zdz, 2) && tma_ok(sigA, CS) && (NSIG == 1 || tma_ok(sigB, CS)))) return 1;
     BilateralTmaParams p{};
     p.r = 2 * (int)ceilf(sigma * 2.5f) + 1;

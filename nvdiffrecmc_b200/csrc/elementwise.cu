@@ -10,8 +10,11 @@
 // coalesced), broadcast operands (e.g. view_pos [B,1,1,3]) fall back to strided scalar loads that
 // hit L1; grid = enough 256-thread CTAs to cover the pixels (>= several waves over 148 SMs at
 // 512x512), no shared memory, no divergence except the BSDF's own branches.
+// A cp.async.bulk + mbarrier pipeline that staged the contiguous operands in shared memory was measured on B200 and was slower on
+// every op (pbr_bsdf 16x512^2 fwd 0.107 vs 0.094 ms, bwd 0.309 vs 0.213 ms; shade tail fwd 0.033 vs 0.031 ms): these ops are
+// instruction-issue / dependency bound (385-860 instructions per pixel at 94-139 registers), and the stages cost occupancy.  It was
+// removed; the evidence is in profiles/r02_ew_tma_ab.json.
 #include "bsdf.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -20,13 +23,11 @@ struct Grid { int N, H, W; int64_t npx; };
 struct TIn {
     TView v;
     int fast;      // contiguous, full grid, 16B aligned -> vector path
-    int sm_off;    // >= 0: byte offset of this operand inside a shared-memory stage of the bulk-copy pipeline (ew_kernel_tma); -1: not staged
 };
 
 struct Px4 {
     int64_t p0;
     int cnt;
-    const unsigned char *stage;   // shared-memory stage holding this tile's staged operands, or nullptr (direct global loads)
 };
 
 __device__ __forceinline__ void px_decode(const Grid &g, int64_t p, int &n, int &h, int &w)
@@ -43,15 +44,11 @@ template <int C, bool FULL>
 __device__ __forceinline__ void ew_load(const TIn &t, const Grid &g, const Px4 &q, float (&out)[4][C])
 {
     if (FULL && t.fast) {
-        // staged tile: thread t owns bytes [t * 16 C, (t + 1) * 16 C) of the operand's slab -- 128-bit shared loads, conflict-free for
-        // C = 1, 3 (a quarter warp covers 8 x 16 C bytes: distinct banks for odd C); otherwise 128-bit read-only global loads
-        const bool staged = q.stage != nullptr && t.sm_off >= 0;
-        const float4 *src = staged ? reinterpret_cast<const float4 *>(q.stage + t.sm_off) + (size_t)threadIdx.x * C
-                                   : reinterpret_cast<const float4 *>(t.v.p + q.p0 * C);
+        const float4 *src = reinterpret_cast<const float4 *>(t.v.p + q.p0 * C);
         float buf[4 * C];
 #pragma unroll
         for (int i = 0; i < C; ++i) {
-            float4 x = staged ? src[i] : __ldg(src + i);
+            float4 x = __ldg(src + i);
             buf[4 * i + 0] = x.x; buf[4 * i + 1] = x.y; buf[4 * i + 2] = x.z; buf[4 * i + 3] = x.w;
         }
 #pragma unroll
@@ -100,113 +97,18 @@ __device__ __forceinline__ void ew_store(float *dst, const Px4 &q, const float (
 __device__ __forceinline__ f3 to3(const float (&a)[3]) { return F3(a[0], a[1], a[2]); }
 __device__ __forceinline__ void from3(float (&a)[3], f3 v) { a[0] = v.x; a[1] = v.y; a[2] = v.z; }
 
-#ifndef MCS_EW_MINB
-#define MCS_EW_MINB 2          // caps the heaviest op (pbr_bsdf backward, 139 regs) at 128 so two CTAs fit: 0.32 -> 0.21 ms at 16x512x512
-#endif
+constexpr int EW_MINB = 2;     // caps the heaviest op (pbr_bsdf backward, 139 regs) at 128 so two CTAs fit: 0.32 -> 0.21 ms at 16x512x512
 template <class Op>
-__global__ void __launch_bounds__(256, MCS_EW_MINB) ew_kernel(Op op, Grid g)
+__global__ void __launch_bounds__(256, EW_MINB) ew_kernel(Op op, Grid g)
 {
     int64_t q4 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     Px4 q;
     q.p0 = q4 * 4;
-    q.stage = nullptr;
     if (q.p0 >= g.npx) return;
     int64_t rem = g.npx - q.p0;
     q.cnt = rem >= 4 ? 4 : (int)rem;
     if (q.cnt == 4) op.template run<true>(g, q);
     else op.template run<false>(g, q);
-}
-
-// ---------------------------------------------------------------------------------------------
-// Bulk-copy (TMA) pipeline for the heavy streaming ops -- OPT-IN (MCS_EW_TMA=1), see launch_tma() for the measured verdict. (pbr_bsdf, prepare_shading_normal, the shade() tail; forward and backward).
-// ncu on the direct-load kernel (profiles/r01_secondary_ncu_summary.json): 44 % DRAM / 47 % issue at 94-139 registers -- every warp
-// first waits for its own 18-21 128-bit loads, then computes, then stores, and with 16 warps per SM nothing overlaps the two.
-// Here the loads leave the warps entirely: persistent CTAs walk the tiles of 4 * EW_TMA_THREADS pixels; ONE thread per CTA issues, per
-// tile and per contiguous operand, one 1-D `cp.async.bulk.shared::cluster.global` (SASS UBLKCP) of the operand's slab into a
-// shared-memory stage, completion counted in bytes on an mbarrier; the tile after next is in flight while the current one is
-// computed from shared memory with the same per-thread code as before (ew_load reads 128-bit shared words instead of global ones).
-// Broadcast / strided operands (view_pos [B,1,1,3]) are not staged and keep the scalar path; the ragged last tile takes the direct
-// path.  Results go out with 128-bit global stores straight from registers.
-// ---------------------------------------------------------------------------------------------
-#ifndef EW_TMA_THREADS
-#define EW_TMA_THREADS 128
-#endif
-#ifndef EW_TMA_STAGES
-#define EW_TMA_STAGES 2
-#endif
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, int count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count)); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
-{
-    asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra DONE_%=;\nbra WAIT_%=;\nDONE_%=:\n}" ::"r"(smem_u32(bar)),
-                 "r"(parity)
-                 : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)), "l"(src), "r"(bytes),
-                 "r"(smem_u32(bar))
-                 : "memory");
-}
-
-template <class Op>
-__global__ void __launch_bounds__(EW_TMA_THREADS) ew_kernel_tma(Op op, Grid g, int64_t ntiles, int64_t nfull, uint32_t stage_bytes)
-{
-    extern __shared__ __align__(128) unsigned char ew_smem[];
-    __shared__ __align__(8) uint64_t full[EW_TMA_STAGES];
-    constexpr int TPX = EW_TMA_THREADS * 4;
-    const int tid = threadIdx.x;
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < EW_TMA_STAGES; ++s) mbar_init(&full[s], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    auto issue = [&](int64_t tile, int s) {      // thread 0 only: arm the stage's barrier with the byte count, then one bulk copy per operand
-        mbar_expect_tx(&full[s], stage_bytes);
-#pragma unroll
-        for (int i = 0; i < Op::NIN; ++i) {
-            const TIn &t = op.in(i);
-            if (t.sm_off >= 0) {
-                const uint32_t bytes = (uint32_t)(TPX * sizeof(float)) * (uint32_t)t.v.n3;
-                bulk_g2s(ew_smem + (size_t)s * stage_bytes + t.sm_off, t.v.p + tile * TPX * t.v.n3, bytes, &full[s]);
-            }
-        }
-    };
-    if (tid == 0) {
-#pragma unroll
-        for (int k = 0; k < EW_TMA_STAGES - 1; ++k) {
-            const int64_t t0 = (int64_t)blockIdx.x + (int64_t)k * gridDim.x;
-            if (t0 < nfull) issue(t0, k);
-        }
-    }
-    int it = 0;
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-        const int s = it % EW_TMA_STAGES;
-        if (tid == 0) {       // the stage consumed in the previous iteration is free (barrier below): refill it with the tile after next
-            const int64_t nt = tile + (int64_t)(EW_TMA_STAGES - 1) * gridDim.x;
-            if (nt < nfull) issue(nt, (it + EW_TMA_STAGES - 1) % EW_TMA_STAGES);
-        }
-        Px4 q;
-        q.p0 = tile * TPX + (int64_t)tid * 4;
-        if (tile < nfull) {
-            mbar_wait(&full[s], (uint32_t)((it / EW_TMA_STAGES) & 1));
-            q.cnt = 4;
-            q.stage = ew_smem + (size_t)s * stage_bytes;
-            op.template run<true>(g, q);
-        } else if (q.p0 < g.npx) {                // ragged last tile: direct loads
-            const int64_t rem = g.npx - q.p0;
-            q.cnt = rem >= 4 ? 4 : (int)rem;
-            q.stage = nullptr;
-            if (q.cnt == 4) op.template run<true>(g, q);
-            else op.template run<false>(g, q);
-        }
-        __syncthreads();
-    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -374,9 +276,6 @@ struct SpecBwd {
     }
 };
 struct PbrFwd {
-    static constexpr int NIN = 6;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&kd, &arm, &pos, &nrm, &view, &light}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&kd, &arm, &pos, &nrm, &view, &light}; return *a[i]; }
     TIn kd, arm, pos, nrm, view, light; float min_roughness; int bsdf; float *out;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
     {
@@ -390,9 +289,6 @@ struct PbrFwd {
     }
 };
 struct PbrBwd {
-    static constexpr int NIN = 7;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&kd, &arm, &pos, &nrm, &view, &light, &dout}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&kd, &arm, &pos, &nrm, &view, &light, &dout}; return *a[i]; }
     TIn kd, arm, pos, nrm, view, light, dout; float min_roughness; int bsdf;
     float *d_kd, *d_arm, *d_pos, *d_nrm, *d_view, *d_light;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
@@ -413,9 +309,6 @@ struct PbrBwd {
     }
 };
 struct PsnFwd {
-    static constexpr int NIN = 6;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&pos, &view, &pn, &sn, &st, &gn}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&pos, &view, &pn, &sn, &st, &gn}; return *a[i]; }
     TIn pos, view, pn, sn, st, gn; int two_sided, opengl; float *out;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
     {
@@ -435,9 +328,6 @@ struct PsnFwd {
     }
 };
 struct PsnBwd {
-    static constexpr int NIN = 7;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&pos, &view, &pn, &sn, &st, &gn, &dout}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&pos, &view, &pn, &sn, &st, &gn, &dout}; return *a[i]; }
     TIn pos, view, pn, sn, st, gn, dout; int two_sided, opengl;
     float *d_pos, *d_view, *d_pn, *d_sn, *d_st, *d_gn;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
@@ -479,9 +369,6 @@ struct PsnBwd {
 // the demodulated signals:  shaded = (A.rgb / A.w) * kd * (1 - ks.z) + B.rgb / B.w   ('pbr');   shaded = (A.rgb / A.w) * kd   ('diffuse' / 'white').
 // One launch instead of ~8 torch element-wise kernels forward and ~14 backward.
 struct CombineFwd {
-    static constexpr int NIN = 4;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&a4, &b4, &kd, &ks}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&a4, &b4, &kd, &ks}; return *a[i]; }
     TIn a4, b4, kd, ks; int pbr; float *out;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
     {
@@ -498,9 +385,6 @@ struct CombineFwd {
     }
 };
 struct CombineBwd {
-    static constexpr int NIN = 5;
-    __host__ __device__ const TIn &in(int i) const { const TIn *a[NIN] = {&a4, &b4, &kd, &ks, &dout}; return *a[i]; }
-    __host__ TIn &in_mut(int i) { TIn *a[NIN] = {&a4, &b4, &kd, &ks, &dout}; return *a[i]; }
     TIn a4, b4, kd, ks, dout; int pbr; float *d_a4, *d_b4, *d_kd, *d_ks;
     template <bool FULL> __device__ void run(const Grid &g, const Px4 &q) const
     {
@@ -553,7 +437,6 @@ static bool mk_in(const mcs_tensor *t, const Grid &g, int C, TIn &out, const cha
     bool contig = t->sizes[0] == g.N && t->sizes[1] == g.H && t->sizes[2] == g.W && t->sizes[3] == C &&
                   (C == 1 || t->strides[3] == 1) && t->strides[2] == C && t->strides[1] == C * g.W && t->strides[0] == C * g.W * g.H;
     out.fast = contig && ((uintptr_t)t->ptr % 16 == 0);
-    out.sm_off = -1;
     return true;
 }
 
@@ -566,43 +449,6 @@ static int launch(const Op &op, const Grid &g, cudaStream_t s)
     int64_t nblocks = (nthreads + block - 1) / block;
     MCS_REQUIRE(nblocks < (1ll << 31), "elementwise grid too large");
     ew_kernel<Op><<<(unsigned)nblocks, block, 0, s>>>(op, g);
-    MCS_LAUNCH_CHECK();
-    return 0;
-}
-
-// Bulk-copy pipeline launcher: stage every contiguous operand; fall back to the direct kernel for small problems (fewer tiles than CTAs
-// would leave the pipeline empty) or when nothing can be staged.
-template <class Op>
-static int launch_tma(Op &op, const Grid &g, cudaStream_t s)
-{
-    if (g.npx == 0) return 0;
-    constexpr int TPX = EW_TMA_THREADS * 4;
-    uint32_t stage_bytes = 0;
-    for (int i = 0; i < Op::NIN; ++i) {
-        TIn &t = op.in_mut(i);
-        if (t.fast) { t.sm_off = (int)stage_bytes; stage_bytes += (uint32_t)(TPX * sizeof(float)) * (uint32_t)t.v.n3; }
-    }
-    const int64_t nfull = g.npx / TPX, ntiles = (g.npx + TPX - 1) / TPX;
-    static int sms = 0;
-    if (!sms) { int dev = 0; MCS_CUDA(cudaGetDevice(&dev)); MCS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)); }
-    // Measured on B200 (profiles/r02_ew_tma_ab.json, same library, L2 flushed): the pipeline is CORRECT (GPU parity suite passes with it
-    // forced on) but SLOWER than the direct kernel on every op -- pbr_bsdf 16x512^2 fwd 0.107 vs 0.094 ms, bwd 0.309 vs 0.213 ms; shade
-    // tail fwd 0.033 vs 0.031 ms -- because these ops are instruction-issue / dependency bound (385-860 instructions per pixel at 94-139
-    // registers), not bytes-in-flight bound: the stages cost occupancy (8-12 warps per SM instead of 16) and that outweighs the
-    // overlap.  The direct kernel therefore stays the default; MCS_EW_TMA=1 selects the pipeline (A/B, tests).
-    static const bool enabled = getenv("MCS_EW_TMA") != nullptr;
-    if (!enabled || stage_bytes == 0 || nfull < 2 * (int64_t)sms) {
-        for (int i = 0; i < Op::NIN; ++i) op.in_mut(i).sm_off = -1;
-        return launch(op, g, s);
-    }
-    const size_t smem = (size_t)stage_bytes * EW_TMA_STAGES;
-    int per_sm = 0;
-    MCS_CUDA(cudaFuncSetAttribute(ew_kernel_tma<Op>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MCS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ew_kernel_tma<Op>, EW_TMA_THREADS, smem));
-    if (per_sm < 1) { for (int i = 0; i < Op::NIN; ++i) op.in_mut(i).sm_off = -1; return launch(op, g, s); }
-    const int64_t want = (int64_t)sms * per_sm;
-    const unsigned grid = (unsigned)(ntiles < want ? ntiles : want);
-    ew_kernel_tma<Op><<<grid, EW_TMA_THREADS, smem, s>>>(op, g, ntiles, nfull, stage_bytes);
     MCS_LAUNCH_CHECK();
     return 0;
 }
@@ -702,7 +548,7 @@ int mcs_pbr_bsdf_fwd(const mcs_tensor *kd, const mcs_tensor *arm, const mcs_tens
     GRID(kd, arm, pos, nrm, view_pos, light_pos); PbrFwd op;
     IN(kd, kd, 3); IN(arm, arm, 3); IN(pos, pos, 3); IN(nrm, nrm, 3); IN(view, view_pos, 3); IN(light, light_pos, 3);
     op.min_roughness = min_roughness; op.bsdf = bsdf; op.out = out;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 int mcs_pbr_bsdf_bwd(const mcs_tensor *kd, const mcs_tensor *arm, const mcs_tensor *pos, const mcs_tensor *nrm, const mcs_tensor *view_pos,
                      const mcs_tensor *light_pos, float min_roughness, int32_t bsdf, const mcs_tensor *d_out,
@@ -712,7 +558,7 @@ int mcs_pbr_bsdf_bwd(const mcs_tensor *kd, const mcs_tensor *arm, const mcs_tens
     IN(kd, kd, 3); IN(arm, arm, 3); IN(pos, pos, 3); IN(nrm, nrm, 3); IN(view, view_pos, 3); IN(light, light_pos, 3); IN(dout, d_out, 3);
     op.min_roughness = min_roughness; op.bsdf = bsdf;
     op.d_kd = d_kd; op.d_arm = d_arm; op.d_pos = d_pos; op.d_nrm = d_nrm; op.d_view = d_view_pos; op.d_light = d_light_pos;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 int mcs_prepare_shading_normal_fwd(const mcs_tensor *pos, const mcs_tensor *view_pos, const mcs_tensor *perturbed_nrm, const mcs_tensor *smooth_nrm,
                                    const mcs_tensor *smooth_tng, const mcs_tensor *geom_nrm, int32_t two_sided_shading, int32_t opengl,
@@ -721,7 +567,7 @@ int mcs_prepare_shading_normal_fwd(const mcs_tensor *pos, const mcs_tensor *view
     GRID(pos, view_pos, perturbed_nrm, smooth_nrm, smooth_tng, geom_nrm); PsnFwd op;
     IN(pos, pos, 3); IN(view, view_pos, 3); IN(pn, perturbed_nrm, 3); IN(sn, smooth_nrm, 3); IN(st, smooth_tng, 3); IN(gn, geom_nrm, 3);
     op.two_sided = two_sided_shading; op.opengl = opengl; op.out = out;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 int mcs_prepare_shading_normal_bwd(const mcs_tensor *pos, const mcs_tensor *view_pos, const mcs_tensor *perturbed_nrm, const mcs_tensor *smooth_nrm,
                                    const mcs_tensor *smooth_tng, const mcs_tensor *geom_nrm, int32_t two_sided_shading, int32_t opengl,
@@ -733,20 +579,20 @@ int mcs_prepare_shading_normal_bwd(const mcs_tensor *pos, const mcs_tensor *view
     IN(pos, pos, 3); IN(view, view_pos, 3); IN(pn, perturbed_nrm, 3); IN(sn, smooth_nrm, 3); IN(st, smooth_tng, 3); IN(gn, geom_nrm, 3); IN(dout, d_out, 3);
     op.two_sided = two_sided_shading; op.opengl = opengl;
     op.d_pos = d_pos; op.d_view = d_view_pos; op.d_pn = d_perturbed_nrm; op.d_sn = d_smooth_nrm; op.d_st = d_smooth_tng; op.d_gn = d_geom_nrm;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 
 int mcs_shade_combine_fwd(const mcs_tensor *a4, const mcs_tensor *b4, const mcs_tensor *kd, const mcs_tensor *ks, int32_t pbr, float *out, mcs_stream s)
 {
     GRID(a4, b4, kd, ks); CombineFwd op; IN(a4, a4, 4); IN(b4, b4, 4); IN(kd, kd, 3); IN(ks, ks, 3); op.pbr = pbr; op.out = out;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 int mcs_shade_combine_bwd(const mcs_tensor *a4, const mcs_tensor *b4, const mcs_tensor *kd, const mcs_tensor *ks, int32_t pbr, const mcs_tensor *d_out,
                           float *d_a4, float *d_b4, float *d_kd, float *d_ks, mcs_stream s)
 {
     GRID(a4, b4, kd, ks, d_out); CombineBwd op; IN(a4, a4, 4); IN(b4, b4, 4); IN(kd, kd, 3); IN(ks, ks, 3); IN(dout, d_out, 3); op.pbr = pbr;
     op.d_a4 = d_a4; op.d_b4 = d_b4; op.d_kd = d_kd; op.d_ks = d_ks;
-    return launch_tma(op, gb.g, (cudaStream_t)s);
+    return launch(op, gb.g, (cudaStream_t)s);
 }
 
 }  // extern "C"

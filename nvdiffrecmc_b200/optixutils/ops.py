@@ -143,8 +143,6 @@ class _optix_env_shade_func(torch.autograd.Function):
         hit = rec_cnt = rec_rays = None
         slots = 2 * n_samples_x * n_samples_x
         mode = HIT_RECORD_REPLAY if (rnd_seed is not None and need_grad) else None
-        if mode is True:
-            mode = "bits"
         if mode == "rays" and not _ray_record_fits(B * H * W * (slots * 20 + 4), ro.device):
             mode = "bits"
         if mode == "rays":

@@ -35,15 +35,21 @@ for shape in [(1, 256, 256), (16, 512, 512), (1, 2048, 2048)]:          # test_b
     npx = B * H * W
     t = [torch.rand(B, H, W, 3, generator=g).to(dev) for _ in range(7)]
     kd, arm, pos, nrm, view, light, dout = t
-    ins = [x.clone().requires_grad_(True) for x in (kd, arm, pos, nrm, view, light)]
-    for name, fwd_bytes, bwd_bytes, f in [
-        ("pbr_bsdf", 84, 156, lambda a: ru.pbr_bsdf(a[0], a[1], a[2], a[3], a[4], a[5])),
-        ("prepare_shading_normal", 84, 156, lambda a: ru.prepare_shading_normal(a[2], a[4], a[0], a[3], a[1], a[5], two_sided_shading=True, opengl=True)),
+    rough, dout1 = [torch.rand(B, H, W, 1, generator=g).to(dev) for _ in range(2)]
+    ins = [x.clone().requires_grad_(True) for x in (kd, arm, pos, nrm, view, light, rough)]
+    for name, fwd_bytes, bwd_bytes, used, f in [            # used: indices into ins of the op's differentiable inputs
+        ("pbr_bsdf", 84, 156, range(6), lambda a: ru.pbr_bsdf(a[0], a[1], a[2], a[3], a[4], a[5])),
+        ("prepare_shading_normal", 84, 156, range(6),
+         lambda a: ru.prepare_shading_normal(a[2], a[4], a[0], a[3], a[1], a[5], two_sided_shading=True, opengl=True)),
+        ("pbr_specular", 64, 116, (0, 3, 4, 5, 6), lambda a: ru.pbr_specular(a[0], a[1], a[2], a[3], a[4])),
+        ("frostbite_diffuse", 44, 84, (3, 5, 4, 6), lambda a: ru.frostbite_diffuse(a[0], a[1], a[2], a[3])),
     ]:
+        xs = [ins[i] for i in used]
         with torch.no_grad():
-            ms_f = timed(lambda: f([x.detach() for x in ins]))
-        y = f(ins)
-        ms_b = timed(lambda: torch.autograd.grad(y, ins, dout, retain_graph=True))
+            ms_f = timed(lambda: f([x.detach() for x in xs]))
+        y = f(xs)
+        dy = dout if y.shape[-1] == 3 else dout1
+        ms_b = timed(lambda: torch.autograd.grad(y, xs, dy, retain_graph=True))
         out["ops"].append({"op": name, "shape": list(shape), "fwd_ms": round(ms_f, 4), "fwd_gbs": round(npx * fwd_bytes / ms_f / 1e6, 1),
                            "fwd_frac_of_hbm_peak": round(npx * fwd_bytes / ms_f / 1e6 / peak, 3), "bwd_ms": round(ms_b, 4),
                            "bwd_gbs": round(npx * bwd_bytes / ms_b / 1e6, 1), "bwd_frac_of_hbm_peak": round(npx * bwd_bytes / ms_b / 1e6 / peak, 3),
@@ -85,7 +91,6 @@ colB = torch.rand(B, H, W, 3, generator=g).to(dev)
 with torch.no_grad():
     ms_f2 = timed(lambda: ou.bilateral_denoiser2(col.detach(), colB, nrm, zdz, 2.0))
 out["bilateral_denoiser"] = {"shape": [B, H, W], "sigma": 2.0, "taps_per_px": 529, "fwd_ms": round(ms_f, 4), "fwd2_ms_two_signals": round(ms_f2, 4), "bwd_ms": round(ms_b, 4),
-                             "fwd_path": "plain (MCS_DENOISE_NO_TMA)" if os.environ.get("MCS_DENOISE_NO_TMA") else "TMA-staged",
                              "fwd_gtaps_per_s": round(taps / ms_f / 1e6, 1), "fwd_gbs_compulsory_48B_per_px": round(B * H * W * 48 / ms_f / 1e6, 1)}
 print(out["bilateral_denoiser"], flush=True)
 

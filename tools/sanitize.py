@@ -37,7 +37,7 @@ for N in (4, 9):
     rast = rasterize(ctx, (proj @ mv)[None], (24, 24))
     att = t("verts").clone().requires_grad_(True)
     interpolate(att, rast, t("tris"))[0].sum().backward()
-# round 2: records entry point (MODE 2), fused shade tail, texel fetch, device-side seed, and -- with MCS_EW_TMA=1 -- the bulk-copy pipeline
+# round 2: records entry point (MODE 2), fused shade tail, texel fetch, device-side seed
 from nvdiffrecmc_b200.optixutils.ops import env_shade_records, shade_combine
 from nvdiffrecmc_b200.raster import texel_fetch
 env_shade_records(ctx, t("mask"), t("ro"), t("pos"), nrm.detach(), t("view"), t("kd"), t("ks"), t("light"), t("pdf"), t("rows"), t("cols"), t("perms"), n_samples_x=N, rnd_seed=1)
@@ -47,10 +47,5 @@ a4 = (torch.rand(2, 12, 12, 4, device=dev) + 0.5).requires_grad_(True)
 shade_combine(a4, a4 * 1.5, t("kd"), t("ks")).sum().backward()
 tex = torch.rand(64, 3, device=dev, requires_grad=True)
 texel_fetch(tex, torch.randint(0, 64, (2, 12, 12), device=dev)).sum().backward()
-if os.environ.get("MCS_EW_TMA"):
-    B, H, W = 1, 400, 400          # 160 000 px = 312 tiles of 512 px (>= 2 x 148) + a ragged tail
-    ins = [torch.rand(B, H, W, 3, device=dev).requires_grad_(True) for _ in range(6)]
-    y = ru.pbr_bsdf(*ins); y.sum().backward()
-    n2 = ru.prepare_shading_normal(ins[2], ins[4], ins[0], ins[3], ins[1], ins[5]); n2.sum().backward()
 torch.cuda.synchronize()
 print("sanitize workload ok", float(loss), int(v.sum()), tuple(pts.shape))
